@@ -414,13 +414,52 @@ def reads_roofline(rs, n_reads, target_len, nloc_sum, sm_mhz, peak, peak_src):
                     "8d's accounting (every alignment 'consumes' its whole target), which the exact seed filter does not execute"}
 
 
-def run_reads_workload(E, target, reads, steps, warmup, e2e_n, flush, barrier, want_cpu=None, cpu_seconds=15.0):
-    """One reads-vs-one-target HW distance workload: resident value, e2e, optional CPU sample with parity."""
+def dump_outputs(res, out_dir, prefix="", budget=63 << 20):
+    """Writes what the caller of the timed path received from its last step, one .npy per field: edit_distance and
+    num_locations (float32, one per read), end_locations and start_locations (float64, every location of every read in
+    read order; start_locations only where the task returns them).  Past `budget` bytes of data (under 64 MB with the
+    file headers), the reads are a fixed seeded sample, listed in sample_index.npy."""
+    n = len(res)
+    rows = np.arange(n)
+    order = np.random.Generator(np.random.PCG64(0)).permutation(n)
+    while True:
+        nloc = res["numLocations"][rows].astype(np.int64)
+        starts = bool(res["startLocations"][rows].any())
+        size = len(rows) * (8 + (8 if len(rows) < n else 0)) + int(nloc.sum()) * (16 if starts else 8)
+        if size <= budget or len(rows) <= 1:
+            break
+        rows = np.sort(order[:len(rows) // 2])
+
+    def locations(field):
+        out = np.empty(int(nloc.sum()), dtype=np.float64)
+        at = 0
+        for i, c in zip(rows, nloc):
+            if c:
+                out[at:at + c] = np.frombuffer(C.string_at(int(res[field][i]), 4 * int(c)), dtype=np.int32)
+                at += c
+        return out
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"edit_distance": res["editDistance"][rows].astype(np.float32),
+              "num_locations": nloc.astype(np.float32), "end_locations": locations("endLocations")}
+    if starts:
+        arrays["start_locations"] = locations("startLocations")
+    if len(rows) < n:
+        arrays["sample_index"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
+def run_reads_workload(E, target, reads, steps, warmup, e2e_n, flush, barrier, want_cpu=None, cpu_seconds=15.0, dump=None):
+    """One reads-vs-one-target HW distance workload: resident value, e2e, optional CPU sample with parity.  `dump`:
+    (directory, file prefix) for the results of the last timed step (dump_outputs)."""
     n = reads.shape[0]
     ptrs = pointer_arrays(reads, target)
     cfg, _ = make_config(-1, MODE_HW, TASK_DISTANCE)
     rs = resident_steps(E, ptrs, n, cfg, steps, warmup, flush, barrier)
     res = rs.pop("res")
+    if dump:
+        dump_outputs(res, *dump)
     eds = res["editDistance"].copy()
     nloc = res["numLocations"].copy()
     cpu = None
@@ -757,7 +796,11 @@ def main():
                     help="comma-separated sub-records to run (default: all)")
     ap.add_argument("--config3-pairs", type=int, default=100_000)
     ap.add_argument("--strong-reads", type=int, default=10_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step of the headline workload to DIR/<name>.npy (dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -812,7 +855,8 @@ def main():
         sampler.start()
     rs, ee, eds, nloc, cpu = run_reads_workload(E, target, reads, args.steps, args.warmup, args.e2e_steps, flush_l2, barrier,
                                                 want_cpu=(cores if (rank == 0 and world == 1 and not args.no_cpu_baseline) else None),
-                                                cpu_seconds=args.cpu_seconds)
+                                                cpu_seconds=args.cpu_seconds,
+                                                dump=(args.dump_outputs, "rank%d_" % rank if world > 1 else "") if args.dump_outputs else None)
     all_clocks = sampler.stop() if sampler else {}
     clocks = all_clocks.get(local_rank)
     elapsed = torch.tensor([sum(rs["step_s"])], dtype=torch.float64, device=dev)

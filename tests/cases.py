@@ -291,6 +291,45 @@ KNOWN = [
 ]
 
 
+def hirschberg_cases(seed, count):
+    """PATH of long pairs (query x target beyond the reference's 1 MiB stored-matrix rule, edlib.cpp:1188-1211): short
+    queries in long targets and mutated copies, alphabets of 2, 4 and 10 symbols, every mode."""
+    rng = random.Random(seed)
+    for _ in range(count):
+        alpha = bytes(rng.sample(range(256), rng.choice([2, 4, 10])))
+        if rng.random() < 0.5:
+            q = rand_seq(rng, rng.randrange(50, 350), alpha)
+            t = rand_seq(rng, rng.randrange(9000, 14000), alpha)
+        else:
+            t = rand_seq(rng, rng.randrange(1500, 4000), alpha)
+            q = mutate(rng, t, rng.choice([0.02, 0.2]), alpha)
+        mode = rng.choice([0, 0, 1, 2])
+        yield dict(q=q, t=t, k=-1, mode=mode, task=2, eqs=None)
+
+
+def cigar_scripts(seed, count):
+    """Edit scripts for edlibAlignmentToCigar: every length around the word boundaries, runs of every length, and now
+    and then a bad operation code.  Yields (ops, bad)."""
+    rng = random.Random(seed)
+    for _ in range(count):
+        n = rng.choice([0, 1, 2, 7, 8, 9, 15, 16, 17, 31, 33, 64, 150, 151, 1000, 1500, 5000])
+        style = rng.randrange(4)
+        if style == 0:
+            ops = bytes(rng.choice([0, 0, 0, 0, 0, 0, 1, 2, 3]) for _ in range(n))
+        elif style == 1:
+            ops = bytes([rng.randrange(4)]) * n
+        elif style == 2:
+            ops = b"".join(bytes([rng.randrange(4)]) * rng.randrange(1, 40) for _ in range(n // 8 + 1))[:n]
+        else:
+            ops = bytes(rng.randrange(4) for _ in range(n))
+        bad = rng.random() < 0.03 and n > 0
+        if bad:
+            ops = bytearray(ops)
+            ops[rng.randrange(n)] = rng.choice([4, 7, 255])
+            ops = bytes(ops)
+        yield ops, bad
+
+
 def big_batch_case(seed, num=140_000, target_len=4000):
     """One HW batch large enough for the multi-threaded host paths (classification, seed-stage
     outcomes, end-location assembly): short reads of two word classes over one target, with empty

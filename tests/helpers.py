@@ -1,4 +1,6 @@
 """Test-side wiring: loads the checkers (oracle restatement, reference build) and the product."""
+import hashlib
+import json
 import os
 import random
 
@@ -30,6 +32,23 @@ def product():
     if "product" not in _cache:
         _cache["product"] = EdlibLib(product_path(), prefix="edlib", has_batch=True)
     return _cache["product"]
+
+
+def digest(value):
+    """Short fingerprint of a result dict, a string or None, as stored in tests/golden/ref_digests.json (bytes fields are
+    hashed as hex, dict keys in sorted order)."""
+    if isinstance(value, dict):
+        value = {k: (v.hex() if isinstance(v, bytes) else v) for k, v in value.items()}
+    text = json.dumps(value, sort_keys=True, default=int)
+    return hashlib.sha256(text.encode()).hexdigest()[:8]
+
+
+def golden_digests():
+    """tests/golden/ref_digests.json: fingerprints of the reference build's answers (tests/golden/make_ref_digests.py)."""
+    if "golden" not in _cache:
+        with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_digests.json")) as f:
+            _cache["golden"] = json.load(f)
+    return _cache["golden"]
 
 
 def rand_seq(rng, n, alphabet):

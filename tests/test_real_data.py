@@ -71,20 +71,18 @@ def test_ecoli_all_reads_hw_locations_on_gpu():
 
 def test_phage_nw_distances_config1():
     """BASELINE configs[0] and its siblings: mutated phage genomes vs the phage genome (94 kbp), NW, k = -1
-    (band doubling on the warp kernel): SURVEY.md 8c's measured reference values.  Needs the reference tree."""
-    d = "/root/reference/test_data/Enterobacteria_Phage_1/"
-    if not os.path.exists(d + "Enterobacteria_phage_1.fasta"):
-        pytest.skip("reference test data not present")
+    (band doubling on the warp kernel): SURVEY.md 8c's measured reference values.  The reference's test data travel as
+    tests/golden/phage_nw.fasta.xz (generator tests/golden/make_phage.py)."""
+    import lzma
     from test_engine_emul import load_emul
 
-    def read_fasta(path):
-        with open(path, "rb") as f:
-            return b"".join(l.strip() for l in f if not l.startswith(b">"))
-
-    target = read_fasta(d + "Enterobacteria_phage_1.fasta")
+    with lzma.open(os.path.join(HERE, "golden", "phage_nw.fasta.xz")) as f:
+        lines = f.read().split(b"\n")
+    seqs = dict(zip((l[1:].decode() for l in lines[0::2]), lines[1::2]))
+    target = seqs["Enterobacteria_phage_1"]
     assert len(target) == 94481
     lib = load_emul()
     for pc, ed in ((99, 990), (97, 2977), (94, 6042), (90, 9506)):
-        q = read_fasta(d + "mutated_%d_perc.fasta" % pc)
+        q = seqs["mutated_%d_perc" % pc]
         r = lib.align(q, target, -1, 0, 0)
         assert r["editDistance"] == ed and r["endLocations"] == [94480] and r["startLocations"] is None, (pc, r)

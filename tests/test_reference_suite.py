@@ -38,10 +38,25 @@ def test_reference_runtests_on_gpu():
     assert out.stdout.count("40/40") == 6 and "All specific tests passed!" in out.stdout
 
 
+HELLO = r'''
+#include <stdio.h>
+#include "edlib.h"
+
+int main(void) {
+    EdlibAlignResult r = edlibAlign("hello", 5, "world!", 6, edlibDefaultAlignConfig());
+    printf("status %d, edit distance %d\n", r.status, r.editDistance);
+    edlibFreeAlignResult(r);
+    return r.status;
+}
+'''
+
+
 @pytest.mark.gpu
-def test_reference_hello_world_on_gpu():
-    exe = os.path.join(REFBIN, "helloWorld_b200")
-    if not os.path.exists(exe):
-        pytest.skip("reference example binary did not travel")
+def test_reference_hello_world_on_gpu(tmp_path):
+    """The reference's hello-world example in C: a plain C caller of include/edlib.h, linked against the product library."""
+    exe = str(tmp_path / "hello")
+    lib = os.path.join(REPO, "edlib_b200", "lib")
+    subprocess.run(["gcc", "-x", "c", "-std=c99", "-I", os.path.join(REPO, "include"), "-o", exe, "-", "-L" + lib, "-ledlib_b200",
+                    "-Wl,-rpath," + lib], input=HELLO, text=True, check=True)
     out = subprocess.run([exe], capture_output=True, text=True)
-    assert out.returncode == 0 and "edit_distance('hello', 'world!') = 5" in out.stdout
+    assert out.returncode == 0 and out.stdout == "status 0, edit distance 5\n"

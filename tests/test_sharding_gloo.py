@@ -42,10 +42,10 @@ dist.destroy_process_group()
 '''
 
 
-def test_two_rank_shard_broadcast_gather():
+def test_two_rank_shard_broadcast_gather(tmp_path):
     subprocess.run(["make", "-s", "-C", os.path.join(REPO, "tests", "emul")], check=True)
     subprocess.run(["make", "-s", "-C", os.path.join(REPO, "edlib_b200", "csrc"), "../lib/libsynth.so"], check=True)
-    script = "/tmp/edlib_gloo_worker.py"
+    script = str(tmp_path / "edlib_gloo_worker.py")
     with open(script, "w") as f:
         f.write(WORKER % {"repo": REPO})
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
